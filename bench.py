@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the per-ray rendering hot path (BASELINE.json metric: rays/s, fwd+bwd, NeRF-Synthetic-lego shape).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C3|C4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C3|C4] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline (`value`, `e2e`, `roofline`): config C2 = nerf-blender HashGrid L16/F2/T2^19 + FullyFused-64 fields, 8192 rays per GPU.
@@ -17,6 +17,9 @@ At N = 1 the same JSON line also carries
   * `cpu_baseline`: BASELINE.json config 1 -- the reference's own pure-torch fields (VanillaFrequency + VanillaMLP, 4096 rays) inside
     the CPU oracle's marching / compositing, fwd+bwd on the host cores; `cpu_baseline_secondary`: the fp32 CPU port of C2 itself.
 `--impl reference` times the CPU port of the headline config on the host cores at the SAME rays per step it reports.
+`--dump-outputs DIR` (GPU headline only, rank 0) writes what the last timed step handed its caller to DIR/<name>.npy: `loss`, the
+per-ray float outputs, `num_samples` and `grad.<parameter name>` for every trainable parameter.  Inputs are seeded, so two builds run with
+the same arguments can be compared array by array.
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
 """
 import argparse
@@ -242,6 +245,28 @@ def build_model(device, seed=0):
     return model
 
 
+DUMP_MAX_ELEMS = 1 << 22   # larger arrays are dumped as a fixed seeded sample of this many entries: a whole dump stays well under 64 MB
+
+
+def snapshot_outputs(loss, out, named_params, n_rays):
+    """device copies of what one step returns to its caller: the loss, the per-ray float outputs (the capacity-length per-sample buffers
+    are undefined past num_samples and laid out in allocation order, so they are left out), the kept-sample count, every gradient"""
+    snap = {'loss': loss, 'num_samples': out['num_samples_dev'] if 'num_samples_dev' in out else out['num_samples']}
+    snap.update({k: v for k, v in out.items() if torch.is_tensor(v) and v.is_floating_point() and v.dim() >= 1 and v.shape[0] == n_rays})
+    snap.update({f'grad.{name}': p.grad for name, p in named_params if p.requires_grad and p.grad is not None})
+    return {k: v.detach().clone() for k, v in snap.items()}
+
+
+def write_outputs(dirname, snap):
+    os.makedirs(dirname, exist_ok=True)
+    for name, v in snap.items():
+        if v.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(v.numel(), DUMP_MAX_ELEMS, replace=False))
+            v = v.reshape(-1)[torch.from_numpy(idx).to(v.device)]
+        v = v.float() if v.is_floating_point() and v.dtype != torch.float64 else v.double()
+        np.save(os.path.join(dirname, f'{name}.npy'), v.cpu().numpy())
+
+
 def masked_smooth_l1(comp_rgb, target, valid):
     """systems/nerf.py:97 without the host sync of boolean indexing: mean over valid rays x 3 channels."""
     m = valid.float()
@@ -249,13 +274,13 @@ def masked_smooth_l1(comp_rgb, target, valid):
     return per.sum() / (m.sum() * 3.0).clamp(min=1.0)
 
 
-def neus_config(name, dev, steps, warmup, flush, peak, peak_src):
+def neus_config(name, dev, steps, warmup, flush, peak, peak_src, dump=None):
     """BASELINE.json config 3 (neus-blender with mask, 8192 rays; static-shape step = one CUDA graph) or config 4 (neus-dtu with learned
     background, 4096 rays; eager: the background pass has host-sized outputs) on one GPU: fwd + the reference's loss terms
     (systems/neus.py:98-121 as nsr_b200.losses.neus_losses) + bwd.  Returns a sub-line: rays/s (median of per-step CUDA events, L2
     flushed before every step), e2e (pinned host rays / targets / masks in, loss scalar out), per-kernel times and the roofline of the
     dominant kernel.  Synthetic scene as SURVEY 8d: sphere-init SDF, occupancy = shell around the surface (+ a 15 % random background
-    grid for C4), seeded rays, cos_anneal_ratio 0.25."""
+    grid for C4), seeded rays, cos_anneal_ratio 0.25.  ``dump``: a dict that receives snapshot_outputs() of the last timed step."""
     from nsr_b200 import models, configs, synthetic
     from nsr_b200.lib import lib
     from nsr_b200.losses import neus_losses
@@ -314,11 +339,13 @@ def neus_config(name, dev, steps, warmup, flush, peak, peak_src):
         flush.fill_(float(i))
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        step(rays_dev[j], tgt_dev[j], msk_dev[j])
+        loss = step(rays_dev[j], tgt_dev[j], msk_dev[j])
         e1.record()
         evs.append((e0, e1))
     torch.cuda.synchronize()
     launches = lib.launches
+    if dump is not None:
+        dump.update(snapshot_outputs(loss, gs.out if graphed else step.last, m.named_parameters(), n))
     per = [a.elapsed_time(b) for a, b in evs]
     host = []
     for i in range(steps):
@@ -402,8 +429,11 @@ def neus_arm(args):
     peak, peak_src = peaks()
     sampler = ClockSampler(0)
     sampler.start()
-    sub = neus_config(args.config, dev, args.steps, max(3, args.warmup), flush, peak, peak_src)
+    dump = {} if args.dump_outputs else None
+    sub = neus_config(args.config, dev, args.steps, max(3, args.warmup), flush, peak, peak_src, dump=dump)
     clocks = sampler.stop()
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     line = dict(sub)
     line.update({'n_gpus': 1, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'data': 'synthetic', 'clocks': clocks})
     sys.stdout.flush()
@@ -528,6 +558,7 @@ def gpu_arm(args):
     per_step = timed(args.steps, e2e=False)
     barrier()
     launches = lib.launches
+    dump = snapshot_outputs(gstep.loss, gstep.out, model.named_parameters(), N_RAYS) if args.dump_outputs and rank == 0 else None
     # ---- end-to-end: pinned host buffers in, loss out, same K steps
     barrier()
     per_step_e2e = timed(args.steps, e2e=True)
@@ -702,6 +733,8 @@ def gpu_arm(args):
                                                     f"fp32 CPU oracle, {cpu['cores']} threads"}
     if extra:
         line['extra'] = extra
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)
     print(json.dumps(line), flush=True)
@@ -719,7 +752,12 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--config', default='C2', choices=['C2', 'C3', 'C4'], help='headline config (C3 / C4: single GPU)')
     ap.add_argument('--no-extra', action='store_true', help='skip the C3 / C4 sub-lines of the default run')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs and gradients of the last timed step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the GPU path (--impl ours)')
     if args.impl == 'reference':
         reference_arm(args)
     elif args.config == 'C2':

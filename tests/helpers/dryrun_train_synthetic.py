@@ -4,7 +4,7 @@ process only: tcnn modules and nerfacc-shaped functions by the oracle-backed sta
 by oracle/rays.py, the fused losses by oracle/losses.py, FusedAdamW by torch.optim.AdamW, the occupancy refresh by a full grid."""
 import sys, os, types, importlib.util, json, time
 import numpy as np, torch
-ROOT='/root/repo'; sys.path.insert(0, ROOT); sys.path.insert(0, ROOT+'/tests/helpers')
+ROOT=os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))); sys.path.insert(0, ROOT); sys.path.insert(0, ROOT+'/tests/helpers')
 import cpu_thirdparty as tp
 from nsr_b200 import models as ours, tcnn as our_tcnn, rays as nrays, optim as noptim, configs
 from nsr_b200.models import nerf_model, neus_model

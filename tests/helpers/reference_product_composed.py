@@ -1,7 +1,9 @@
 """Run in a subprocess by tests/test_reference_dropin.py.  The PRODUCT's drop-in models (nsr_b200.models 'nerf' / 'neus') executed on the
 CPU through their composed (per-op) code path -- the CUDA-backed tcnn modules swapped for the oracle-backed stand-ins and the nerfacc-shaped
 functions rebound to the stand-ins (tests/helpers/cpu_thirdparty.py) -- against the UNMODIFIED reference models built on the same stand-ins
-with the same weights: the Python orchestration of the drop-in models (everything that is not a kernel) for C2, C3 and C4."""
+with the same weights: the Python orchestration of the drop-in models (everything that is not a kernel) for C2, C3 and C4.  The original
+models' weights, outputs and gradients are stored in tests/golden/reference_product_composed.npz (tests/helpers/golden_ref.py;
+``--record DIR`` re-creates it)."""
 import contextlib
 import json
 import os
@@ -12,9 +14,9 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = '/root/reference'
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from golden_ref import Tape, pick, amax, is_array  # noqa: E402
 
 
 def _stub(name, **attrs):
@@ -25,6 +27,7 @@ def _stub(name, **attrs):
 
 
 def main():
+    T = Tape('reference_product_composed')
     import cpu_thirdparty as tp
     from nsr_b200.config import Config, to_primitive
     from nsr_b200 import configs, synthetic, models as ours, tcnn as our_tcnn
@@ -54,8 +57,9 @@ def main():
     sysm = _stub('systems')
     sysm.utils = _stub('systems.utils', update_module_step=lambda m, e, s: m.update_step(e, s) if hasattr(m, 'update_step') else None)
     torch.cuda.device = lambda idx: contextlib.nullcontext()
-    sys.path.insert(0, REF)
-    import models as ref_models
+    if T.recording:
+        sys.path.insert(0, T.reference)
+        import models as ref_models
 
     # the product's nerfacc-shaped entry points -> CPU stand-ins (only inside this process)
     for mod in (nerf_model, neus_model):
@@ -76,7 +80,8 @@ def main():
                 swap_tcnn(child)
 
     def mx(a, b):
-        a, b = torch.as_tensor(a).detach().double().reshape(-1), torch.as_tensor(b).detach().double().reshape(-1)
+        a, b = pick(a, b)
+        a, b = a.double(), b.double()
         assert a.shape == b.shape, (a.shape, b.shape)
         return float((a - b).abs().max()) if a.numel() else 0.0
 
@@ -91,16 +96,20 @@ def main():
         cfg['fused'] = False
         if 'geometry' in cfg:
             cfg['geometry']['fused'] = False
+        name = f'{kind}:{cfg_fn.__name__}'
         torch.manual_seed(0)
-        ref = ref_models.make(kind, Config(cfg_fn() | {'randomized': False}))
         our = ours.make(kind, cfg)
         swap_tcnn(our)
-        prepare(ref)
-        our.load_state_dict(ref.state_dict(), strict=True)
+        prepare(our)
+        if T.recording:   # the unmodified reference model with our weights
+            ref = ref_models.make(kind, Config(cfg_fn() | {'randomized': False}))
+            missing, unexpected = ref.load_state_dict(our.state_dict(), strict=False)   # (the stand-in grid has no grid_coords / grid_indices)
+            assert not missing and all('occupancy_grid' in k for k in unexpected), (missing, unexpected)
+        T.check_state(our, f'{name}/state')
         r = rays.copy()
         r[:, :3] *= ray_scale
-        outs, grads = [], []
-        for m in (our, ref):
+
+        def run_model(m):
             m.train()
             m.update_step(0, 5001)            # not a multiple of 16: the product's occupancy refresh needs CUDA
             m.background_color = bg
@@ -108,22 +117,22 @@ def main():
                 p.grad = None
             out = m.forward_(torch.from_numpy(r))
             loss_fn(out).backward()
-            outs.append(out)
-            grads.append({k: p.grad.clone() for k, p in m.named_parameters() if p.grad is not None})
-        a, b = outs
+            grads = {k: p.grad.clone() for k, p in m.named_parameters() if p.grad is not None}
+            # eval mode: chunked, detached, parked on the CPU, plus inv_s for NeuS
+            m.eval()
+            with torch.no_grad():
+                ev = m(torch.from_numpy(r))
+            return {k: v.detach() if torch.is_tensor(v) else v for k, v in out.items()}, grads, ev
+        a, ga, ea = run_model(our)
+        b, gb, eb = T.ref(f'{name}/run', lambda: run_model(ref))
         entry = {'keys_equal': sorted(a) == sorted(b), 'only_ours': sorted(set(a) - set(b)), 'only_ref': sorted(set(b) - set(a)),
-                 'num_samples': int(b['num_samples']), 'diff': {k: mx(a[k].float(), b[k].float()) for k in b if torch.is_tensor(b[k])},
-                 'dtype_equal': all(a[k].dtype == b[k].dtype for k in b if torch.is_tensor(b[k]) and k in a),
-                 'grad_keys_equal': sorted(grads[0]) == sorted(grads[1]),
-                 'grad_diff': max(mx(grads[0][k], grads[1][k]) / (float(grads[1][k].abs().max()) + 1e-30) for k in grads[1] if k in grads[0])}
-        # eval mode: chunked, detached, parked on the CPU, plus inv_s for NeuS
-        our.eval()
-        ref.eval()
-        with torch.no_grad():
-            ea, eb = our(torch.from_numpy(r)), ref(torch.from_numpy(r))
+                 'num_samples': int(b['num_samples']), 'diff': {k: mx(a[k].float(), b[k]) for k in b if is_array(b[k])},
+                 'dtype_equal': all(a[k].dtype == b[k].dtype for k in b if is_array(b[k]) and k in a),
+                 'grad_keys_equal': sorted(ga) == sorted(gb),
+                 'grad_diff': max(mx(ga[k], gb[k]) / (amax(gb[k]) + 1e-30) for k in gb if k in ga)}
         entry['eval_keys_equal'] = sorted(ea) == sorted(eb)
-        entry['eval_diff'] = max(mx(ea[k].float(), eb[k].float()) for k in eb if torch.is_tensor(eb[k]) and k in ea)
-        res[f'{kind}:{cfg_fn.__name__}'] = entry
+        entry['eval_diff'] = max(mx(ea[k].float(), eb[k]) for k in eb if is_array(eb[k]) and k in ea)
+        res[name] = entry
 
     def prep_nerf(m):
         from nsr_b200 import ops
@@ -172,6 +181,8 @@ def main():
         ray_scale=1.0 / 1.5 * 0.4)
     run('neus', configs.neus_blender, prep_neus, neus_loss)
     run('neus', configs.neus_dtu, prep_dtu, neus_loss, ray_scale=1.0 / 1.5 * 0.6)
+    if T.recording:
+        T.save()
     print('RESULT ' + json.dumps(res))
 
 

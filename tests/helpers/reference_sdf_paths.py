@@ -2,7 +2,8 @@
 normals through autograd when the fused kernel is off, finite-difference normals + laplacian with the ProgressiveBandHashGrid of the
 Neuralangelo config) executed on the CPU -- their hash-grid encoding swapped for the oracle-backed stand-in
 (tests/helpers/cpu_thirdparty.py) -- against the reference's own VolumeSDF (models/geometry.py:141-238) built on the same stand-in with the
-same weights."""
+same weights.  The original's values are stored in tests/golden/reference_sdf_paths.npz (tests/helpers/golden_ref.py; ``--record DIR``
+re-creates it)."""
 import contextlib
 import json
 import os
@@ -12,9 +13,9 @@ import types
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = '/root/reference'
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from golden_ref import Tape, pick, amax  # noqa: E402
 
 
 def _stub(name, **attrs):
@@ -25,6 +26,7 @@ def _stub(name, **attrs):
 
 
 def main():
+    T = Tape('reference_sdf_paths')
     import cpu_thirdparty as tp
     from nsr_b200.config import Config, to_primitive
     from nsr_b200 import configs
@@ -53,22 +55,21 @@ def main():
     sysm = _stub('systems')
     sysm.utils = _stub('systems.utils', update_module_step=lambda m, e, s: m.update_step(e, s) if hasattr(m, 'update_step') else None)
     torch.cuda.device = lambda idx: contextlib.nullcontext()
-    sys.path.insert(0, REF)
-    import models as ref_models                      # noqa: F401  (registers the reference classes)
-    from models import geometry as rgeo, network_utils as rnet
-    rnet.get_rank = lambda: 'cpu'                    # ProgressiveBandHashGrid allocates its mask on device=get_rank()
+    if T.recording:
+        sys.path.insert(0, T.reference)
+        import models as ref_models                      # noqa: F401  (registers the reference classes)
+        from models import geometry as rgeo, network_utils as rnet
+        rnet.get_rank = lambda: 'cpu'                    # ProgressiveBandHashGrid allocates its mask on device=get_rank()
     from nsr_b200.models import fields as ofields
     from nsr_b200.nerfacc import ContractionType as OurCT
 
     res = {}
 
     def mx(a, b):
-        return float((a.detach().double() - b.detach().double()).abs().max())
+        a, b = pick(a, b)
+        return float((a.double() - b.double()).abs().max())
 
-    def pair(geo_cfg, steps):
-        torch.manual_seed(0)
-        ref = rgeo.VolumeSDF(Config(geo_cfg))
-        ref.contraction_type = tp.ContractionType.AABB
+    def pair(name, geo_cfg, steps):
         torch.manual_seed(0)
         our = ofields.VolumeSDF(Config(geo_cfg))
         our.contraction_type = OurCT.AABB
@@ -80,47 +81,65 @@ def main():
         else:
             our.encoding.encoding = tp.Encoding(3, grid_cfg)
         with torch.no_grad():
-            v = ref.network.layers[0].weight_v if hasattr(ref.network.layers[0], 'weight_v') else ref.network.layers[0].weight
+            v = our.network.layers[0].weight_v if hasattr(our.network.layers[0], 'weight_v') else our.network.layers[0].weight
             v[:, 3:] = torch.randn(v.shape[0], v.shape[1] - 3) * 0.05
-        missing = our.load_state_dict(ref.state_dict(), strict=True)
+        if T.recording:   # the reference's VolumeSDF on the same stand-in, with our weights
+            torch.manual_seed(0)
+            ref = rgeo.VolumeSDF(Config(geo_cfg))
+            ref.contraction_type = tp.ContractionType.AABB
+            ref.load_state_dict(our.state_dict(), strict=True)
+        T.check_state(our, f'{name}/state')
         out = {}
         pts = (torch.rand(300, 3, generator=torch.Generator().manual_seed(1)) * 2 - 1) * 0.8 * geo_cfg['radius']
         for step in steps:
             for mode in ('train', 'eval'):
-                getattr(ref, mode)()
                 getattr(our, mode)()
-                ref.update_step(0, step)
                 our.update_step(0, step)
                 fd = geo_cfg['grad_type'] == 'finite_difference'
                 a = our(pts.clone(), with_grad=True, with_feature=True, with_laplace=fd)
-                b = ref(pts.clone(), with_grad=True, with_feature=True, with_laplace=fd)
-                names = ['sdf', 'grad', 'feature'] + (['laplace'] if fd else [])
-                d = {n: mx(x, y) for n, x, y in zip(names, a, b)}
-                d['level'] = mx(our.forward_level(pts), ref.forward_level(pts))
-                d['sdf_only'] = mx(our(pts.clone(), with_grad=False, with_feature=False), ref(pts.clone(), with_grad=False, with_feature=False))
-                if mode == 'train':   # eikonal-style loss through the normals: second-order path of the torch fallback
-                    for mod, o in ((our, a), (ref, b)):
-                        for p in mod.parameters():
+
+                def ref_run():
+                    getattr(ref, mode)()
+                    ref.update_step(0, step)
+                    b = ref(pts.clone(), with_grad=True, with_feature=True, with_laplace=fd)
+                    r = {'out': [x.detach() for x in b], 'level': ref.forward_level(pts).detach(),
+                         'sdf_only': ref(pts.clone(), with_grad=False, with_feature=False).detach()}
+                    if mode == 'train':
+                        for p in ref.parameters():
                             p.grad = None
-                        (((o[1].norm(dim=-1) - 1) ** 2).mean() + o[0].mean()).backward()
-                    go, gr = dict(our.named_parameters()), dict(ref.named_parameters())
-                    d['param_grad'] = max(mx(go[k].grad, gr[k].grad) / (float(gr[k].grad.abs().max()) + 1e-30) for k in gr if gr[k].grad is not None)
-                    d['requires_grad_outputs'] = float(a[0].requires_grad != b[0].requires_grad)
+                        (((b[1].norm(dim=-1) - 1) ** 2).mean() + b[0].mean()).backward()
+                        r['param_grad'] = {k: p.grad for k, p in ref.named_parameters() if p.grad is not None}
+                        r['requires_grad'] = b[0].requires_grad
+                    return r
+                b = T.ref(f'{name}/{step}/{mode}', ref_run)
+                names = ['sdf', 'grad', 'feature'] + (['laplace'] if fd else [])
+                d = {n: mx(x, y) for n, x, y in zip(names, a, b['out'])}
+                d['level'] = mx(our.forward_level(pts), b['level'])
+                d['sdf_only'] = mx(our(pts.clone(), with_grad=False, with_feature=False), b['sdf_only'])
+                if mode == 'train':   # eikonal-style loss through the normals: second-order path of the torch fallback
+                    for p in our.parameters():
+                        p.grad = None
+                    (((a[1].norm(dim=-1) - 1) ** 2).mean() + a[0].mean()).backward()
+                    go, gr = dict(our.named_parameters()), b['param_grad']
+                    d['param_grad'] = max(mx(go[k].grad, gr[k]) / (amax(gr[k]) + 1e-30) for k in gr)
+                    d['requires_grad_outputs'] = float(a[0].requires_grad != b['requires_grad'])
                 else:
                     d['detached'] = float(any(t.requires_grad for t in a))
                 out[f'{step}/{mode}'] = d
         return out
 
     na = configs.neuralangelo_dtu()['geometry']
-    res['finite_difference_progressive'] = pair(na, (0, 2500, 20000))
+    res['finite_difference_progressive'] = pair('finite_difference_progressive', na, (0, 2500, 20000))
     an = configs.neus_blender()['geometry']
     an['fused'] = False                              # the torch fallback of the analytic-normal path
-    res['analytic_fallback'] = pair(an, (0,))
+    res['analytic_fallback'] = pair('analytic_fallback', an, (0,))
     fixed = dict(configs.neus_blender()['geometry'], grad_type='finite_difference', finite_difference_eps=0.01)
-    res['finite_difference_fixed_eps'] = pair(fixed, (0,))
+    res['finite_difference_fixed_eps'] = pair('finite_difference_fixed_eps', fixed, (0,))
     colmap = dict(configs.neuralangelo_dtu()['geometry'], grad_type='analytic', radius=0.6)   # neus-colmap.yaml: progressive grid + analytic normals
     colmap.pop('finite_difference_eps', None)
-    res['analytic_progressive'] = pair(colmap, (0, 3500))
+    res['analytic_progressive'] = pair('analytic_progressive', colmap, (0, 3500))
+    if T.recording:
+        T.save()
     print('RESULT ' + json.dumps(res))
 
 

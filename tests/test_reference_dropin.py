@@ -1,7 +1,8 @@
-"""Drop-in check at INTEGRATION.md level 1: the UNMODIFIED reference models (/root/reference/models/*.py) import ``tinycudann`` and
+"""Drop-in check at INTEGRATION.md level 1: the UNMODIFIED reference models (instant-nsr-pl's models/*.py) import ``tinycudann`` and
 ``nerfacc`` and get nsr_b200's modules; they construct with the reference's own configs, expose the parameter counts SURVEY.md 8a
 states, share state_dict keys / shapes with the drop-in models (checkpoints load both ways) and refuse CPU tensors the way
-nerfacc 0.3.3 / tiny-cuda-nn do.  Needs /root/reference (present in the build container, absent on the GPU box => skipped there)."""
+nerfacc 0.3.3 / tiny-cuda-nn do.  What the reference computes is stored under tests/golden/ (tests/helpers/golden_ref.py: each helper
+re-creates its file with ``--record <instant-nsr-pl checkout>``), so these tests need nothing outside the repository."""
 import json
 import os
 import subprocess
@@ -12,7 +13,6 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/models'), reason='/root/reference is not mounted here')
 def test_reference_models_build_on_our_modules():
     r = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'helpers', 'reference_dropin.py')], capture_output=True, text=True,
                        timeout=600)
@@ -34,7 +34,6 @@ def test_reference_models_build_on_our_modules():
     assert dtu['n_params'] == dtu['n_params_ours'] and dtu['tcnn_modules'] == ['Encoding']  # neus-dtu: VanillaMLPs everywhere
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/models'), reason='/root/reference is not mounted here')
 def test_oracle_orchestration_is_pinned_to_the_reference_forward():
     """oracle/models.py (nerf_render, neus_render, neus_bg_render, neus_dtu_render) restates models/nerf.py:61-127 and models/neus.py:141-287.  Here the reference's
     OWN forward_ runs on the CPU -- tinycudann / nerfacc replaced by per-op stand-ins built from the oracle's primitives
@@ -70,7 +69,6 @@ def test_oracle_orchestration_is_pinned_to_the_reference_forward():
     assert dtu['occ_fn_bg'] < 1e-6 and dtu['occ_thre'] == [0.001, 0.01]       # the background grid keeps the default threshold
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/systems'), reason='/root/reference is not mounted here')
 def test_oracle_front_end_and_losses_are_pinned_to_the_reference_training_step():
     """The reference's OWN systems/nerf.py / systems/neus.py ``preprocess_data`` and ``training_step`` run on the CPU (tiny in-memory
     dataset, fake model; tests/helpers/reference_system.py): the batch they assemble equals oracle.rays.training_batch / image_batch (the
@@ -100,13 +98,17 @@ def test_oracle_front_end_and_losses_are_pinned_to_the_reference_training_step()
         m = e['mesh']
         assert e['mesh_name'] == 'it3-mc20.obj' and set(m) == {'v_pos', 't_pos_idx', 'v_rgb'}
         assert m['v_pos'][0] > 500 and m['v_pos'] == m['v_rgb'] and m['t_pos_idx'][1] == 3
+        # the same steps restated from the oracle pieces pinned above, on the same drop-in model, reproduce what the systems reported
+        r = e['restated']
+        assert r['train_num_rays'] == e['train_num_rays'] and r['val_grid'] == e['val_grid'] and r['mesh_name'] == e['mesh_name'], (kind, r)
+        assert max(abs(a - b) / abs(b) for a, b in zip(r['losses'], e['losses'])) < 1e-5 and abs(r['val_psnr'] - e['val_psnr']) < 1e-4, (kind, r)
+        assert r['mesh'] == e['mesh'], (kind, r['mesh'])
     # optim.parse_optimizer builds the reference's param groups (same tensors, names, hyper-parameters) around FusedAdamW
     opt = res['optimizer']
     assert opt['ref_class'] == 'AdamW' and opt['our_class'] == 'FusedAdamW' and opt['n_groups'] == 5
     assert opt['names_equal'] and opt['hyper_equal'] and opt['same_tensors']
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/models'), reason='/root/reference is not mounted here')
 def test_product_torch_side_equals_the_reference_functions():
     """every pure-torch piece of the drop-in models compared DIRECTLY with the reference's own (tests/helpers/reference_torch_parts.py):
     activations (value + gradient), scale_anything, contraction, chunk_batch, VanillaFrequency mask schedule, VanillaMLP / tcnn sphere
@@ -127,7 +129,6 @@ def test_product_torch_side_equals_the_reference_functions():
         assert worst(section) == 0.0, (name, section)
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/models'), reason='/root/reference is not mounted here')
 def test_product_volume_sdf_torch_paths_equal_the_reference():
     """VolumeSDF paths of the product that are torch code rather than kernels -- finite-difference normals + laplacian under the
     ProgressiveBandHashGrid schedule (configs/neuralangelo-dtu-wmask.yaml), fixed-eps finite differences, the autograd fallback of the
@@ -147,7 +148,6 @@ def test_product_volume_sdf_torch_paths_equal_the_reference():
                 assert v <= tol, (section, case, name, v)
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/models'), reason='/root/reference is not mounted here')
 def test_product_models_composed_path_equals_the_reference_models_on_cpu():
     """The drop-in 'nerf' / 'neus' models run their per-op (composed) code path on the CPU -- tcnn modules swapped for the oracle-backed
     stand-ins, nerfacc-shaped functions rebound to them (tests/helpers/reference_product_composed.py) -- against the unmodified reference
