@@ -101,7 +101,7 @@ struct RaysBwdArgs {
   const float* g_weights;  // [cap] (loose layout) or NULL
   float* grad_dparams;
   float* grad_cparams;
-  const float* amax;       // device scalar: bound on |dL/dw| (loss-scale selection)
+  const float* amax;       // device scalar: bound on |dL/dw| over the kept samples (loss-scale selection)
   uint32_t* ticket;        // ray queue head (zero on entry)
   float step, loss_scale;
   int64_t n_rays;
@@ -395,20 +395,32 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) nerf_rays_bwd_kernel(con
   }
 }
 
-// bound on |dL/dw_i| over all rays (loss-scale selection): max_r ( |g_rgb|_1 + |g_op| + |g_depth| * t_bound )
+// bound on |dL/dw_i| over the kept samples of all rays (loss-scale selection); rgb lies in [0, 1], so
+//     |dL/dw_i| <= |g_rgb|_1 + |g_op| + |g_depth| * t_bound + |g_weights_i|
+// One warp per ray.  g_weights is read over the ray's kept prefix only: past it the loose buffer is undefined in the static form.
 __global__ void rays_grad_amax_kernel(const float* __restrict__ g_rgb, const float* __restrict__ g_op, const float* __restrict__ g_depth,
-                                      float t_bound, float* __restrict__ amax, int64_t n) {
+                                      const float* __restrict__ g_weights, const int64_t* __restrict__ offsets_m,
+                                      const int32_t* __restrict__ kept, float t_bound, float* __restrict__ amax, int64_t n) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
   float v = 0.f;
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    float b = 0.f;
+  for (int64_t i = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += warps) {
+    const int k = __ldg(kept + i);
+    if (k <= 0) continue;
+    float gw = 0.f;
+    if (g_weights) {
+      const int64_t base = offsets_m[i];
+      for (int j = lane; j < k; j += 32) gw = fmaxf(gw, fabsf(g_weights[base + j]));
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) gw = fmaxf(gw, __shfl_xor_sync(0xffffffffu, gw, o));
+    }
+    float b = gw;
     if (g_rgb) b += fabsf(g_rgb[i * 3]) + fabsf(g_rgb[i * 3 + 1]) + fabsf(g_rgb[i * 3 + 2]);
     if (g_op) b += fabsf(g_op[i]);
     if (g_depth) b += fabsf(g_depth[i]) * t_bound;
     v = fmaxf(v, b);
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  if ((threadIdx.x & 31) == 0 && v > 0.f && isfinite(v)) atomicMax(reinterpret_cast<int*>(amax), __float_as_int(v));
+  if (lane == 0 && v > 0.f && isfinite(v)) atomicMax(reinterpret_cast<int*>(amax), __float_as_int(v));
 }
 
 }  // namespace
@@ -435,7 +447,8 @@ extern "C" int nsr_nerf_rays_bwd(const nsr_nerf_t* f, const float* rays, const f
     attr_set = true;
   }
   if (loss_scale <= 0.f) {
-    rays_grad_amax_kernel<<<(int)min((int64_t)64, (n_rays + 255) / 256), 256, 0, st>>>(g_rgb, g_opacity, g_depth, t_bound, amax, n_rays);
+    rays_grad_amax_kernel<<<(int)min((int64_t)64, (n_rays + 7) / 8), 256, 0, st>>>(g_rgb, g_opacity, g_depth, g_weights, offsets_m, kept, t_bound,
+                                                                                 amax, n_rays);
     NSR_CHECK_LAUNCH("nsr_nerf_rays_bwd(amax)");
   }
   RaysBwdArgs a;

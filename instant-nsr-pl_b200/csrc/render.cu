@@ -89,7 +89,11 @@ __global__ void __launch_bounds__(kWarps * 32) weight_density_fwd_kernel(const f
     const int64_t i = b + lane;
     const float sd = i < end ? sigmas[i] * (t_ends[i] - t_starts[i]) : 0.f;
     const float incl = warp_incl_sum(sd, lane);
-    const float T = __expf(-(carry + incl - sd));
+    // exclusive sum from the neighbour, not incl - sd: after a sample with a huge sigma * delta (an opaque surface) that difference loses
+    // every earlier term to rounding, and inf - inf is NaN
+    float excl = __shfl_up_sync(0xffffffffu, incl, 1);
+    if (lane == 0) excl = 0.f;
+    const float T = __expf(-(carry + excl));
     if (i < end) {
       weights[i] = T * (1.f - __expf(-sd));
       if (trans) trans[i] = T;
@@ -113,7 +117,9 @@ __global__ void __launch_bounds__(kWarps * 32) weight_density_bwd_kernel(const f
     const float w = ok ? weights[i] : 0.f, g = ok ? grad_weights[i] : 0.f;
     const float gw = g * w;
     const float suf = warp_suffix_sum(gw, lane);  // includes own
-    if (ok) grad_sigmas[i] = (t_ends[i] - t_starts[i]) * (g * (trans[i] - w) - (carry + suf - gw));
+    float after = __shfl_down_sync(0xffffffffu, suf, 1);  // sum over the later lanes (suf - gw cancels when g_i w_i dominates it)
+    if (lane == 31) after = 0.f;
+    if (ok) grad_sigmas[i] = (t_ends[i] - t_starts[i]) * (g * (trans[i] - w) - (carry + after));
     carry += __shfl_sync(0xffffffffu, suf, 0);
   }
 }
